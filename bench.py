@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the multimodal-fusion block (forward + backward), BASELINE.json metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 Default workload (config.workload): BASELINE.json configs[1] - VisualBERT (visual_bert/pretrain) trunk, 12L/768/12h/3072,
 128 text tokens + 100 regions x 2048 per sample, bf16 compute, dropout 0.1 (train mode), synthetic SampleList,
@@ -25,6 +25,9 @@ Other named configs, one JSON line each, same timing rules (`--workload`):
                  through oracle/ref_loader.py: kind "reference"), else the oracle restatement (kind "port"), fp32, all host
                  threads, on a bounded sample
   --impl reference : times that CPU arm alone, same metric / config / JSON shape.
+  --dump-outputs DIR : after the device-resident timed steps, writes what the last of them computed - the loss and every
+                 parameter gradient - as DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for
+                 output: with the same arguments the weights, inputs and dropout masks are the same from run to run.
 
 N > 1 (torchrun): weak scaling, batch per GPU fixed, gradients of every rank averaged with NCCL all-reduce on
 slices of the flat gradient buffer overlapped with the backward (mmf_b200.ddp).
@@ -60,9 +63,13 @@ def bert_config(hidden, heads, inter, layers, p, **extra):
 
 
 def _ref_available():
+    """the reference's files staged under oracle/_ref by build() (oracle/build_ref.py); the CPU arms load them from there"""
     try:
         from oracle import build_ref
-        return build_ref.build() is not None and build_ref.available() or os.path.isdir("/root/reference/mmf")
+        if not build_ref.available():
+            return False
+        os.environ.setdefault("MMF_REFERENCE_ROOT", build_ref.DST)
+        return True
     except Exception:
         return False
 
@@ -698,6 +705,35 @@ def kept_traffic(wl_name, B):
     return None, None
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor} as <out_dir>/<name>.npy, float32 (a 0-d tensor, the loss, as float64), DUMP_BYTES at most in
+    all.  Each array gets an equal share; one with more elements than its share holds is written as a fixed sample of
+    them instead (flattened, indices drawn with a generator seeded the same for every array), so two runs or two builds
+    store the same positions."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (DUMP_BYTES // len(arrays) - 128) // 4         # 128: the .npy header
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dim() == 0:
+            a = np.asarray(t.double().cpu().numpy())
+        else:
+            if t.numel() > cap:
+                idx = torch.randint(0, t.numel(), (cap,), generator=torch.Generator().manual_seed(0)).to(t.device)
+                t = t.reshape(-1)[idx]
+            a = t.float().cpu().numpy()
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a)
+        total += os.path.getsize(path)
+    assert total <= DUMP_BYTES, total
+    return total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -726,7 +762,13 @@ def main():
                          "one lease); single GPU only")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="launch every kernel of the step eagerly")
     ap.add_argument("--profile", action="store_true", help="device-resident steps only (for ncu launch lists)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and the parameter gradients of the last timed step as DIR/<name>.npy (b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 arm computed")
 
     wl = WORKLOADS[args.workload]()
     if args.graph is None:
@@ -845,7 +887,7 @@ def main():
             flush.zero_()
             a, b_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            step(dev_batch)
+            last_loss = step(dev_batch)
             b_.record()
             evs.append((a, b_))
         barrier()
@@ -854,7 +896,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            step(dev_batch)
+            last_loss = step(dev_batch)
         e1.record()
         barrier()
         ms_total = e0.elapsed_time(e1)
@@ -864,6 +906,10 @@ def main():
     if args.graph:
         launches = graph_launches * args.steps      # replays do not pass through the C ABI: kernels recorded at capture x steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        outs = {"loss": last_loss}
+        outs.update(("grad." + n, p_.grad) for n, p_ in model.named_parameters() if p_.grad is not None)
+        dump_outputs(args.dump_outputs, outs)
     if args.profile:
         if rank == 0:
             print(json.dumps({"profile_run": True, "ms_per_step": ms_total / args.steps, "launches": launches}))

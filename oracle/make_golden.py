@@ -3,9 +3,10 @@
 Runs only in the build container (needs /root/reference):   python -m oracle.make_golden
 Each fixture holds seeded weights (reference state_dict key names), inputs, the reference's outputs
 and the gradients of a fixed random-projection loss  (out * W_rand).sum()  (SURVEY.md 8d: out.sum()
-is degenerate after a final LayerNorm).  Shapes are tiny so the fixtures are a few hundred KB.
+is degenerate after a final LayerNorm).  Shapes are tiny; a fixture over 1 MB is stored in parts (oracle/golden_io.py).
 All modules run in eval mode (dropout off): the reference's RNG stream is not reproducible elsewhere.
 """
+import json
 import os
 import sys
 import types
@@ -14,6 +15,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import golden_io  # noqa: E402
 from oracle import ref_loader as R  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -38,10 +40,8 @@ def _grads(module, names):
 
 
 def _save(name, obj):
-    os.makedirs(OUT, exist_ok=True)
-    path = os.path.join(OUT, name + ".pt")
-    torch.save(obj, path)
-    print("wrote %s (%.1f KB)" % (path, os.path.getsize(path) / 1024))
+    for path in golden_io.save(name, obj, OUT):
+        print("wrote %s (%.1f KB)" % (path, os.path.getsize(path) / 1024))
 
 
 def golden_bert_encoder():
@@ -702,6 +702,27 @@ def golden_models():
     _save("models", out)
 
 
+# the reference YAML files that MODEL_DEFAULTS (mmf_b200/models.py) restates, and those the config-loading test reads
+MODEL_CONFIG_FILES = ["configs/models/visual_bert/defaults.yaml", "configs/models/vilbert/defaults.yaml",
+                      "configs/models/mmbt/defaults.yaml", "configs/models/mmf_transformer/defaults.yaml",
+                      "configs/models/visual_bert/classification.yaml", "configs/models/mmbt/classification.yaml",
+                      "configs/models/mmbt/with_features.yaml"]
+
+
+def golden_model_configs():
+    """The parsed documents (yaml.safe_load, nothing resolved) of MODEL_CONFIG_FILES, keyed by their path under mmf/."""
+    import yaml
+    docs = {}
+    for rel in MODEL_CONFIG_FILES:
+        with open(os.path.join(R.REF_ROOT, "mmf", rel)) as fh:
+            docs[rel] = yaml.safe_load(fh)
+    path = os.path.join(OUT, "model_configs.json")
+    with open(path, "w") as fh:
+        json.dump(docs, fh, indent=1)
+        fh.write("\n")
+    print("wrote %s" % path)
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(4)
@@ -719,6 +740,7 @@ def main():
     golden_models()
     golden_vit()
     golden_vinvl()
+    golden_model_configs()
 
 
 if __name__ == "__main__":

@@ -48,3 +48,19 @@ def test_kept_traffic_is_reported_only_for_the_batch_it_was_captured_at(bench):
     assert tr is not None and tr > 4e8 and "ncu" in src            # profiles/dominant_traffic.json: 63 MB read + 406 MB written
     assert bench.kept_traffic("visual_bert", 64) == (None, None)
     assert bench.kept_traffic("no_such_workload", 166) == (None, None)
+
+
+def test_dump_outputs_stays_within_its_budget_and_samples_reproducibly(bench, monkeypatch, tmp_path):
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * (128 + 4 * 1000))
+    big = torch.randn(40, 50)
+    arrays = {"loss": torch.tensor(1.25), "grad.small": torch.arange(6.0).reshape(2, 3), "grad.big": big}
+    total = bench.dump_outputs(str(tmp_path / "a"), arrays)
+    assert total <= bench.DUMP_BYTES
+    loss, small, sample = (np.load(tmp_path / "a" / (n + ".npy")) for n in ("loss", "grad.small", "grad.big"))
+    assert loss.dtype == np.float64 and loss.shape == () and float(loss) == 1.25
+    assert small.dtype == np.float32 and np.array_equal(small, np.arange(6.0).reshape(2, 3))
+    assert sample.dtype == np.float32 and sample.shape == (1000,) and np.isin(sample, big.numpy()).all()
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    assert np.array_equal(np.load(tmp_path / "b" / "grad.big.npy"), sample)

@@ -3,16 +3,15 @@
   (2) the oracle run in fp32 on the same device with the same bf16-rounded weights, at config-2 shapes.
 Tolerances: per BASELINE.md 5 the bf16 bar is 1e-2 per layer against the fp32 oracle; end-to-end the reference's own
 bf16-vs-fp32 drift is 1.25e-2 (outputs) / 1.8e-2 (gradients) at 12 layers, which is the bound used for deep stacks."""
-import os
 import types
 
 import pytest
 import torch
 
 from oracle import fusion_oracle as O
+from oracle import golden_io
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def rel(a, b, floor=1e-3):
@@ -53,7 +52,7 @@ def bert_cfg(hidden, heads, inter, layers, p=0.0):
 
 def test_bert_encoder_vs_reference_golden():
     from mmf_b200.modules import B200BertEncoder
-    g = torch.load(os.path.join(GOLD, "bert_encoder.pt"), weights_only=False)
+    g = golden_io.load("bert_encoder")
     c = g["cfg"]
     enc = B200BertEncoder(bert_cfg(c["hidden"], c["heads"], c["inter"], c["layers"]))
     assert set(enc.state_dict().keys()) == set(g["state_dict"].keys())  # checkpoint-key compatibility
@@ -74,7 +73,7 @@ def test_bert_encoder_vs_reference_golden():
 
 def test_vilbert_encoder_vs_reference_golden():
     from mmf_b200.modules import B200ViLBertEncoder
-    g = torch.load(os.path.join(GOLD, "vilbert_encoder.pt"), weights_only=False)
+    g = golden_io.load("vilbert_encoder")
     c = dict(g["cfg"])
     cfg = types.SimpleNamespace(hidden_dropout_prob=0.0, v_hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0,
                                 v_attention_probs_dropout_prob=0.0, **c)

@@ -1,13 +1,13 @@
 """SURVEY.md 8a row a13 on the GPU: the ReLU GEMM epilogue + its backward, the fc7 region-feature encoder and the
-TransformerEncoder wrapper against the reference's own outputs (tests/golden/encoders.pt), incl. the padding_idx
+TransformerEncoder wrapper against the reference's own outputs (tests/golden/encoders.*.pt), incl. the padding_idx
 rule of HF word embeddings (the [PAD] row is read but gets no gradient)."""
-import os
 
 import pytest
 import torch
 
+from oracle import golden_io
+
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def rel(a, b, floor=1e-3):
@@ -16,7 +16,7 @@ def rel(a, b, floor=1e-3):
 
 
 def gold():
-    return torch.load(os.path.join(GOLD, "encoders.pt"), weights_only=False)
+    return golden_io.load("encoders")
 
 
 @pytest.mark.parametrize("M,N,K", [(300, 128, 256), (1000, 2048, 2048), (77, 264, 72)])

@@ -10,6 +10,7 @@ import torch
 
 from mmf_b200 import engine as E
 from oracle import fusion_oracle as O
+from oracle import golden_io
 
 import fake_kernels as FK
 
@@ -152,9 +153,6 @@ def test_vilbert_connection_layer_wiring_matches_oracle(fake):
 # the drop-in modules end to end (autograd Function, parameter pack hand-over, ViLBERT schedule) over the test double,
 # against the reference's own outputs (tests/golden)
 # ---------------------------------------------------------------------------------------------------------------
-import os
-
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 @pytest.fixture()
@@ -170,7 +168,7 @@ def _golden_bound(e, tol=4e-2):
 
 
 def test_bert_encoder_module_vs_reference_golden_cpu(cpu_modules):
-    g = torch.load(os.path.join(GOLD, "bert_encoder.pt"), weights_only=False)
+    g = golden_io.load("bert_encoder")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0,
@@ -215,7 +213,7 @@ def test_bert_encoder_applied_twice_in_one_graph_cpu(cpu_modules):
 
 
 def test_vilbert_encoder_module_vs_reference_golden_cpu(cpu_modules):
-    g = torch.load(os.path.join(GOLD, "vilbert_encoder.pt"), weights_only=False)
+    g = golden_io.load("vilbert_encoder")
     cfg = types.SimpleNamespace(hidden_dropout_prob=0.0, v_hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0,
                                 v_attention_probs_dropout_prob=0.0, **dict(g["cfg"]))
     enc = cpu_modules.B200ViLBertEncoder(cfg)
@@ -293,7 +291,7 @@ def cpu_frontends(cpu_modules, monkeypatch):
 
 
 def test_visio_linguistic_embeddings_vs_reference_golden_cpu(cpu_frontends):
-    g = torch.load(os.path.join(GOLD, "embeddings.pt"), weights_only=False)
+    g = golden_io.load("embeddings")
     sd = g["vl_state_dict"]
     cfg = types.SimpleNamespace(hidden_size=sd["word_embeddings.weight"].shape[1],
                                 vocab_size=sd["word_embeddings.weight"].shape[0],
@@ -319,7 +317,7 @@ def test_visio_linguistic_embeddings_vs_reference_golden_cpu(cpu_frontends):
 
 
 def test_mmbt_vs_reference_golden_cpu(cpu_frontends):
-    g = torch.load(os.path.join(GOLD, "mmbt.pt"), weights_only=False)
+    g = golden_io.load("mmbt")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], hidden_dropout_prob=0.1, attention_probs_dropout_prob=0.1,
@@ -336,7 +334,7 @@ def test_mmbt_vs_reference_golden_cpu(cpu_frontends):
 
 
 def test_encoder_plugins_vs_reference_golden_cpu(cpu_frontends):
-    g = torch.load(os.path.join(GOLD, "encoders.pt"), weights_only=False)
+    g = golden_io.load("encoders")
     f = g["fc7"]
     fc7 = cpu_frontends.EN.B200FinetuneFasterRcnnFpnFc7({"in_dim": 256, "out_dim": 128})
     fc7.load_state_dict(f["state_dict"])
@@ -367,7 +365,7 @@ def test_encoder_plugins_vs_reference_golden_cpu(cpu_frontends):
 
 def test_mmft_backend_and_vilbert_image_embeddings_vs_reference_golden_cpu(cpu_frontends):
     from mmf_b200.registry import registry
-    g = torch.load(os.path.join(GOLD, "mmft_embeddings.pt"), weights_only=False)
+    g = golden_io.load("mmft_embeddings")
     tcfg = types.SimpleNamespace(hidden_size=64, num_attention_heads=1, intermediate_size=128, num_hidden_layers=1,
                                  hidden_dropout_prob=0.1, attention_probs_dropout_prob=0.1, layer_norm_eps=1e-12,
                                  hidden_act="gelu", initializer_range=0.02, vocab_size=50, max_position_embeddings=32,
@@ -383,7 +381,7 @@ def test_mmft_backend_and_vilbert_image_embeddings_vs_reference_golden_cpu(cpu_f
     assert torch.equal(backend.generate_attention_mask(list(g["masks"])), g["attention_mask"])
     seq, first = backend(g["tokens"], g["pos"], g["seg"], list(g["masks"]))
     assert seq.shape == (2, 11, 64) and torch.isfinite(seq.float()).all()
-    ge = torch.load(os.path.join(GOLD, "embeddings.pt"), weights_only=False)
+    ge = golden_io.load("embeddings")
     mod = cpu_frontends.VB.B200ImageFeatureEmbeddings(
         types.SimpleNamespace(v_feature_size=40, v_hidden_size=96, hidden_dropout_prob=0.1))
     mod.load_state_dict(ge["img_state_dict"])
@@ -448,7 +446,7 @@ def test_visual_bert_trunk_vs_oracle_cpu(cpu_frontends):
 def test_uniter_model_base_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
     import mmf_b200.uniter as UN
     monkeypatch.setattr(UN, "_require_cuda", lambda t, what: None)
-    g = torch.load(os.path.join(GOLD, "uniter.pt"), weights_only=False)
+    g = golden_io.load("uniter")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],
@@ -487,7 +485,7 @@ def test_lxmert_encoder_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
     its weight gradients are the sum of the two uses (engine.xlayer_bwd accumulates both into the same regions)."""
     import mmf_b200.lxmert as LX
     monkeypatch.setattr(LX, "_require_cuda", lambda t, what: None)
-    g = torch.load(os.path.join(GOLD, "lxmert.pt"), weights_only=False)
+    g = golden_io.load("lxmert")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0, visual_feat_dim=c["feat_dim"],
@@ -513,7 +511,7 @@ def test_masked_lm_head_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
     loss over all positions == loss over the labelled rows only"""
     import mmf_b200.heads as HD
     monkeypatch.setattr(HD, "_require_cuda", lambda t, what: None)
-    g = torch.load(os.path.join(GOLD, "mlm_head.pt"), weights_only=False)
+    g = golden_io.load("mlm_head")
     cfg = types.SimpleNamespace(hidden_size=g["cfg"]["hidden"], vocab_size=g["cfg"]["vocab"], layer_norm_eps=1e-12,
                                 initializer_range=0.02)
     emb = torch.nn.Embedding(cfg.vocab_size, cfg.hidden_size)
@@ -611,7 +609,7 @@ def test_visual_bert_for_pretraining_vs_oracle_cpu(cpu_frontends, monkeypatch):
 
 def test_visual_bert_bypass_transformer_vs_reference_golden_cpu(cpu_frontends):
     from mmf_b200.visual_bert import B200VisualBERTBase
-    g = torch.load(os.path.join(GOLD, "visual_bert_bypass.pt"), weights_only=False)
+    g = golden_io.load("visual_bert_bypass")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],
@@ -679,7 +677,7 @@ def test_vit_model_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
     projection as a GEMM over unfolded patches, [CLS] + position table, final LayerNorm, pooler) vs mmf/modules/vit.py"""
     import mmf_b200.vit as VT
     monkeypatch.setattr(VT, "_require_cuda", lambda t, what: None)
-    g = torch.load(os.path.join(GOLD, "vit.pt"), weights_only=False)
+    g = golden_io.load("vit")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0,
@@ -728,7 +726,7 @@ def test_vit_model_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
 def test_vinvl_base_vs_reference_golden_cpu(cpu_frontends, monkeypatch):
     import mmf_b200.vinvl as VV
     monkeypatch.setattr(VV, "_require_cuda", lambda t, what: None)
-    g = torch.load(os.path.join(GOLD, "vinvl.pt"), weights_only=False)
+    g = golden_io.load("vinvl")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],

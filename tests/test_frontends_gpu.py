@@ -1,15 +1,14 @@
 """MMBT, MMFTransformer backend, ViLBERT image embeddings and the monkey-patch swap on the GPU, against the
 reference's own outputs (tests/golden) and oracle gradients."""
-import os
 import types
 
 import pytest
 import torch
 
 from oracle import fusion_oracle as O
+from oracle import golden_io
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def rel(a, b, floor=1e-3):
@@ -27,7 +26,7 @@ def bert_cfg(hidden, heads, inter, layers, **kw):
 
 def test_mmbt_vs_reference_golden_and_integer_paths():
     from mmf_b200.mmbt import B200MMBTBase
-    g = torch.load(os.path.join(GOLD, "mmbt.pt"), weights_only=False)
+    g = golden_io.load("mmbt")
     c = g["cfg"]
     base = B200MMBTBase(bert_cfg(c["hidden"], c["heads"], c["inter"], c["layers"], modal_hidden_size=c["modal_hidden"]))
     sd = base.mmbt.state_dict()
@@ -114,7 +113,7 @@ def test_mmbt_backward_vs_oracle():
 def test_mmft_backend_vs_reference_golden():
     from mmf_b200.mmft_backend import B200TransformerBackend
     from mmf_b200.registry import registry
-    g = torch.load(os.path.join(GOLD, "mmft_embeddings.pt"), weights_only=False)
+    g = golden_io.load("mmft_embeddings")
     tcfg = bert_cfg(64, 1, 128, 1, max_position_embeddings=32, pad_token_id=0)
     mods = [dict(type="text", key="text", position_dim=32, embedding_dim=64, segment_id=0),
             dict(type="image", key="image", position_dim=16, embedding_dim=40, segment_id=1)]
@@ -138,7 +137,7 @@ def test_mmft_backend_vs_reference_golden():
 
 def test_vilbert_image_embeddings_vs_reference_golden():
     from mmf_b200.vilbert import B200ImageFeatureEmbeddings
-    g = torch.load(os.path.join(GOLD, "embeddings.pt"), weights_only=False)
+    g = golden_io.load("embeddings")
     mod = B200ImageFeatureEmbeddings(types.SimpleNamespace(v_feature_size=40, v_hidden_size=96, hidden_dropout_prob=0.1))
     assert set(mod.state_dict().keys()) == set(g["img_state_dict"].keys())
     mod.load_state_dict(g["img_state_dict"])

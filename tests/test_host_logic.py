@@ -1,12 +1,11 @@
 """CPU tests of the host-side logic (no GPU compute): C-ABI export, parameter pack, schedules, key names."""
 import ctypes
-import os
 import types
 
 import pytest
 import torch
 
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
+from oracle import golden_io
 
 
 def test_library_loads_and_exports_every_declared_symbol():
@@ -101,7 +100,7 @@ def test_vilbert_schedule_matches_oracle():
 
 def test_state_dict_keys_match_reference_modules():
     from mmf_b200.modules import B200BertEncoder, B200ViLBertEncoder
-    g = torch.load(os.path.join(GOLD, "bert_encoder.pt"), weights_only=False)
+    g = golden_io.load("bert_encoder")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], hidden_dropout_prob=0.1,
@@ -109,7 +108,7 @@ def test_state_dict_keys_match_reference_modules():
     enc = B200BertEncoder(cfg)
     assert {k: tuple(v.shape) for k, v in enc.state_dict().items()} == {k: tuple(v.shape) for k, v in
                                                                         g["state_dict"].items()}
-    g = torch.load(os.path.join(GOLD, "vilbert_encoder.pt"), weights_only=False)
+    g = golden_io.load("vilbert_encoder")
     cfg = types.SimpleNamespace(hidden_dropout_prob=0.1, v_hidden_dropout_prob=0.1, attention_probs_dropout_prob=0.1,
                                 v_attention_probs_dropout_prob=0.1, **g["cfg"])
     enc = B200ViLBertEncoder(cfg)
@@ -164,7 +163,7 @@ def test_encoder_plugins_registered_with_reference_names_and_keys():
     assert registry.get_encoder_class("finetune_faster_rcnn_fpn_fc7") is enc.B200FinetuneFasterRcnnFpnFc7
     assert registry.get_encoder_class("identity") is enc.B200IdentityEncoder
     assert registry.get_encoder_class("transformer") is enc.B200TransformerEncoder
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "encoders.pt"), weights_only=False)
+    g = golden_io.load("encoders")
     c = g["transformer"]["cfg"]
     te = enc.B200TransformerEncoder(dict(hidden_size=c["hidden"], num_hidden_layers=c["layers"],
                                          num_attention_heads=c["heads"], intermediate_size=c["inter"],
@@ -231,7 +230,7 @@ def test_patch_and_undo_restore_forward():
 def test_mmbt_token_surgery_matches_reference_golden_cpu():
     """integer path of MMBTBase.extract_modal_end_token is pure torch integer code: bit-exact on CPU too"""
     from mmf_b200.mmbt import extract_modal_end_token
-    g = torch.load(os.path.join(GOLD, "mmbt.pt"), weights_only=False)
+    g = golden_io.load("mmbt")
     sl = {"input_ids": g["ids"].clone(), "input_mask": g["mask"].clone()}
     end = extract_modal_end_token(sl)
     assert torch.equal(end, g["end_token"])

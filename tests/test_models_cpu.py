@@ -1,6 +1,6 @@
 """Model plugins (mmf_b200.models: registered `visual_bert` / `vilbert` / `mmbt`, SURVEY.md 8b 4th boundary form) on the CPU:
 the host code (config handling, SampleList plumbing with its integer tensors, heads, loss wiring) runs over the kernel
-test double (tests/fake_kernels.py) and is held to tests/golden/models.pt - outputs of the REFERENCE's own registered model
+test double (tests/fake_kernels.py) and is held to tests/golden/models.*.pt - outputs of the REFERENCE's own registered model
 classes (oracle/make_golden.py::golden_models).  The kernels themselves are covered on the GPU (tests/test_models_gpu.py)."""
 import os
 import sys
@@ -11,9 +11,9 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import fake_kernels as FK  # noqa: E402
+from oracle import golden_io  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REF = "/root/reference/mmf"
 
 
 def rel(a, b):
@@ -66,7 +66,7 @@ def _load(model, golden_sd):
                                   "visual_bert_pretraining_default"])
 def test_visual_bert_registered_model_vs_reference(cpu_models, case):
     MD = cpu_models
-    g = torch.load(os.path.join(GOLD, "models.pt"), weights_only=False)
+    g = golden_io.load("models")
     c = g[case]
     cfg = MD.load_model_config("visual_bert", overrides={k: v for k, v in c["config"].items()})
     cfg.losses = [{"type": "cross_entropy"}]
@@ -104,7 +104,7 @@ def test_visual_bert_registered_model_vs_reference(cpu_models, case):
 @pytest.mark.parametrize("head", ["classification", "pretraining"])
 def test_vilbert_registered_model_vs_reference(cpu_models, head):
     MD = cpu_models
-    g = torch.load(os.path.join(GOLD, "models.pt"), weights_only=False)
+    g = golden_io.load("models")
     c = g["vilbert_" + head]
     cfg = MD.load_model_config("vilbert", overrides=dict(c["config"]))
     cfg.losses = [{"type": "cross_entropy"}]
@@ -159,7 +159,7 @@ def test_mmbt_registered_model_classification_runs_and_matches_oracle(cpu_models
     for p in model.parameters():        # bf16-representable weights: the double computes in bf16 like the kernels
         p.data = p.data.to(torch.bfloat16).float()
     from mmf_b200.sample import SampleList
-    g = torch.load(os.path.join(GOLD, "mmbt.pt"), weights_only=False)
+    g = golden_io.load("mmbt")
     sl = SampleList(input_ids=g["ids"].clone(), input_mask=g["mask"].clone(), segment_ids=g["seg"].clone(),
                     image_feature_0=g["feats"].clone(), targets=torch.tensor([1, 0]), dataset_name="hm", dataset_type="val")
     out = model(sl)
@@ -175,10 +175,26 @@ def test_mmbt_registered_model_classification_runs_and_matches_oracle(cpu_models
     assert rel(out["scores"], ref) < 3e-2
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box)")
-def test_restated_defaults_equal_the_reference_yaml(cpu_models):
+@pytest.fixture()
+def reference_configs(tmp_path):
+    """the reference's model YAML files (tests/golden/model_configs.json: their parsed documents, written back as YAML)
+    under a stand-in mmf root"""
+    import json
+
+    import yaml
+    with open(os.path.join(GOLD, "model_configs.json")) as fh:
+        docs = json.load(fh)
+    for relpath, doc in docs.items():
+        path = tmp_path / relpath
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text(yaml.safe_dump(doc, sort_keys=False))
+    return str(tmp_path)
+
+
+def test_restated_defaults_equal_the_reference_yaml(cpu_models, reference_configs):
     """MODEL_DEFAULTS is a restatement: pin it to the YAML files it cites, read with the module's own YAML loader"""
     MD = cpu_models
+    REF = reference_configs
     import mmf_b200.mmft  # noqa: F401  (adds the mmf_transformer defaults)
     for name, rel_path in (("visual_bert", "configs/models/visual_bert/defaults.yaml"),
                            ("vilbert", "configs/models/vilbert/defaults.yaml"), ("mmbt", "configs/models/mmbt/defaults.yaml"),

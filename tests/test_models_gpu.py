@@ -1,13 +1,13 @@
 """Registered model plugins on the B200 (through the C ABI): `forward(SampleList) -> scores / losses` of visual_bert and
-vilbert against the outputs of the REFERENCE's own registered model classes (tests/golden/models.pt), integer tensors with
+vilbert against the outputs of the REFERENCE's own registered model classes (tests/golden/models.*.pt), integer tensors with
 torch.equal, gradients of the heads and of trunk weights against the reference's autograd."""
-import os
 
 import pytest
 import torch
 
+from oracle import golden_io
+
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def rel(a, b):
@@ -29,7 +29,7 @@ def _sample_list(g, dev):
 def test_visual_bert_registered_model(case):
     from mmf_b200 import lib, models as MD
     dev = torch.device("cuda", 0)
-    g = torch.load(os.path.join(GOLD, "models.pt"), weights_only=False)
+    g = golden_io.load("models")
     c = g[case]
     cfg = MD.load_model_config("visual_bert", overrides=dict(c["config"]))
     cfg.losses = [{"type": "cross_entropy"}]
@@ -63,7 +63,7 @@ def test_visual_bert_registered_model(case):
 def test_vilbert_registered_model(head):
     from mmf_b200 import models as MD
     dev = torch.device("cuda", 0)
-    g = torch.load(os.path.join(GOLD, "models.pt"), weights_only=False)
+    g = golden_io.load("models")
     c = g["vilbert_" + head]
     cfg = MD.load_model_config("vilbert", overrides=dict(c["config"]))
     cfg.losses = [{"type": "cross_entropy"}]

@@ -3,10 +3,11 @@ fused AdamW kernel, the UNITER trunk, the LXMERT encoder (shared cross-attention
 bypass_transformer path - against goldens produced by the reference's own files / the oracle.  (These ran behind
 MMFB_STAGED_TESTS in round 1; they are part of the default `-m gpu` suite now.)"""
 import math
-import os
 
 import pytest
 import torch
+
+from oracle import golden_io
 
 pytestmark = pytest.mark.gpu
 
@@ -54,7 +55,7 @@ def test_uniter_model_base_vs_reference_golden():
     """SURVEY.md 8f item 3 (written after the round's GPU budget was spent; CPU-verified over the kernel test double)"""
     import types
     from mmf_b200.uniter import B200UNITERModelBase
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "uniter.pt"), weights_only=False)
+    g = golden_io.load("uniter")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],
@@ -79,7 +80,7 @@ def test_lxmert_encoder_vs_reference_golden():
     """SURVEY.md 8f item 3: cross-modality layers with the shared cross-attention block (CPU-verified over the test double)"""
     import types
     from mmf_b200.lxmert import B200LXMERTEncoder
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "lxmert.pt"), weights_only=False)
+    g = golden_io.load("lxmert")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0, visual_feat_dim=c["feat_dim"],
@@ -115,7 +116,7 @@ def test_gelu_bwd_kernel_and_masked_lm_head():
     assert ((du.float() - ref).norm() / ref.norm()).item() < 5e-3
     tail = F.gelu_bwd(dh.reshape(-1)[:13].contiguous(), u.reshape(-1)[:13].contiguous())      # scalar tail path
     assert ((tail.float() - ref.reshape(-1)[:13]).abs().max() < 2e-2)
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "mlm_head.pt"), weights_only=False)
+    g = golden_io.load("mlm_head")
     cfg = types.SimpleNamespace(hidden_size=g["cfg"]["hidden"], vocab_size=g["cfg"]["vocab"], layer_norm_eps=1e-12,
                                 initializer_range=0.02)
     cls = B200BertPreTrainingHeads(cfg)
@@ -134,7 +135,7 @@ def test_gelu_bwd_kernel_and_masked_lm_head():
 def test_visual_bert_bypass_transformer_vs_reference_golden():
     import types
     from mmf_b200.visual_bert import B200VisualBERTBase
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "visual_bert_bypass.pt"), weights_only=False)
+    g = golden_io.load("visual_bert_bypass")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],
@@ -156,7 +157,7 @@ def test_vit_pre_ln_model_vs_reference_golden():
     """SURVEY.md 8f item 3 / kernel row K7: pre-LN (ViT) layers on the B200 kernels vs mmf/modules/vit.py (golden)"""
     import types
     from mmf_b200.vit import B200ViTModel
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "vit.pt"), weights_only=False)
+    g = golden_io.load("vit")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0,
@@ -195,7 +196,7 @@ def test_vinvl_base_vs_reference_golden():
     same column padding as VinVL's 2054 (both = 6 mod 8)"""
     import types
     from mmf_b200.vinvl import B200VinVLBase
-    g = torch.load(os.path.join(os.path.dirname(__file__), "golden", "vinvl.pt"), weights_only=False)
+    g = golden_io.load("vinvl")
     c = g["cfg"]
     cfg = types.SimpleNamespace(hidden_size=c["hidden"], num_attention_heads=c["heads"], intermediate_size=c["inter"],
                                 num_hidden_layers=c["layers"], vocab_size=c["vocab"], max_position_embeddings=c["max_pos"],

@@ -2,21 +2,19 @@
 (tests/golden/adamw.pt, generated from mmf/modules/optimizers.py), and B200AdamW's host logic - parameter groups mapped
 onto 8-element blocks of the flat buffers, state views, frozen parameters, parameters outside the packs - over the
 kernel test double (tests/fake_kernels.py)."""
-import os
 import types
 
 import pytest
 import torch
 
 from oracle import fusion_oracle as O
+from oracle import golden_io
 
 import fake_kernels as FK
 
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
-
 
 def test_oracle_adamw_matches_the_reference_arithmetic_bit_for_bit():
-    g = torch.load(os.path.join(GOLD, "adamw.pt"), weights_only=False)
+    g = golden_io.load("adamw")
     assert g["adam_w_is"] == "torch.optim.adamw"        # what optimizers.py:8-14 resolves `adam_w` to in this image
     for mode, fn in (("transformers", O.adamw_step_transformers), ("torch", O.adamw_step_torch)):
         ps = [t.clone() for t in g["init"]]

@@ -1,14 +1,13 @@
 """Embedding front-end (K1) + VisualBERT trunk on the GPU: reference goldens, oracle gradients, integer paths."""
-import os
 import types
 
 import pytest
 import torch
 
 from oracle import fusion_oracle as O
+from oracle import golden_io
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def rel(a, b, floor=1e-3):
@@ -23,7 +22,7 @@ def emb_cfg(H=64, V=50, P=32, F=40, p=0.0):
 
 def test_visio_linguistic_embeddings_vs_reference_golden():
     from mmf_b200.embeddings import B200VisioLinguisticEmbeddings
-    g = torch.load(os.path.join(GOLD, "embeddings.pt"), weights_only=False)
+    g = golden_io.load("embeddings")
     mod = B200VisioLinguisticEmbeddings(emb_cfg())
     assert set(mod.state_dict().keys()) == set(g["vl_state_dict"].keys())
     mod.load_state_dict(g["vl_state_dict"])
