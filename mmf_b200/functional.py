@@ -29,6 +29,16 @@ def _idx_len(idx, M, name):
         raise ValueError("%s must be a contiguous vector of %d indices (one per row), got shape %s" % (name, M, tuple(idx.shape)))
 
 
+def _shape(t, shape, name, contiguous=False):
+    """the kernels take a pointer and a row stride and trust the extents: a buffer smaller than the problem is an
+    out-of-bounds device access (a vector, or a buffer read with an implied stride, must also be contiguous)"""
+    if t is None:
+        return
+    if tuple(t.shape) != tuple(shape) or (contiguous and not t.is_contiguous()):
+        raise ValueError("%s must be %s%s, got shape %s%s" % (name, "a contiguous " if contiguous else "", list(shape),
+                                                               list(t.shape), "" if t.is_contiguous() else " (strided)"))
+
+
 def gemm(a, b, *, a_mn=False, b_mn=False, epi=lib.EPI_BIAS, bias=None, aux=None, drop_mask=None,
          drop_scale=1.0, out=None, out2=None, splits=1, block_n=0, cluster=0):
     """C[M,N] = epi(A[M,K] @ B[N,K]^T) on the tcgen05 GEMM.
@@ -55,7 +65,16 @@ def gemm(a, b, *, a_mn=False, b_mn=False, epi=lib.EPI_BIAS, bias=None, aux=None,
             out = torch.empty(M, N, dtype=torch.bfloat16, device=a.device)
         _req(out, torch.bfloat16, "out")
         if epi == lib.EPI_BIAS_GELU and out2 is None:
-            out2 = torch.empty(M, N, dtype=torch.bfloat16, device=a.device)
+            # the kernel stores C2 with C's row stride: give the default C2 the same one
+            out2 = torch.empty(M, max(out.stride(0), N), dtype=torch.bfloat16, device=a.device)[:, :N]
+    _shape(out, (M, N), "gemm: out")
+    if out2 is not None:
+        _req(out2, torch.bfloat16, "out2")
+        _shape(out2, (M, N), "gemm: out2")
+        if out2.stride(0) != out.stride(0):
+            raise ValueError("gemm: out2 must have the row stride of out (%d), got %d" % (out.stride(0), out2.stride(0)))
+    _shape(bias, (N,), "gemm: bias", contiguous=True)
+    _shape(aux, (M, N), "gemm: aux")
     args = GemmArgs()
     args.A, args.lda, args.a_mn = a.data_ptr(), a.stride(0), int(a_mn)
     args.B, args.ldb, args.b_mn = b.data_ptr(), b.stride(0), int(b_mn)
@@ -65,6 +84,7 @@ def gemm(a, b, *, a_mn=False, b_mn=False, epi=lib.EPI_BIAS, bias=None, aux=None,
     args.aux, args.ldaux = (aux.data_ptr(), aux.stride(0)) if aux is not None else (None, 0)
     if drop_mask is not None:
         _req(drop_mask, torch.int32, "drop_mask")
+        _shape(drop_mask, (M, (N + 31) // 32), "gemm: drop_mask")
         args.drop_mask, args.ldmask = drop_mask.data_ptr(), drop_mask.stride(0)
     args.drop_scale = float(drop_scale)
     args.M, args.N, args.K = M, N, K
@@ -109,6 +129,8 @@ def attention_fwd(q, k, v, B, heads, Sq, Skv, mask=None, drop_mask=None, drop_sc
     a = _attn_args(q, k, v, B, heads, Sq, Skv, mask, drop_mask, drop_scale)
     W = q.shape[-1]
     ctx = out if out is not None else torch.empty(B * Sq, W, dtype=torch.bfloat16, device=q.device)
+    _req(ctx, torch.bfloat16, "out")
+    _shape(ctx, (B * Sq, W), "attention_fwd: out")
     lse2 = torch.empty(B, heads, Sq, dtype=torch.float32, device=q.device)
     a.ctx, a.ldo, a.lse2 = ctx.data_ptr(), ctx.stride(0), lse2.data_ptr()
     ctx_lo = None
@@ -128,15 +150,22 @@ def attention_bwd(dctx, q, k, v, ctx, lse2, B, heads, Sq, Skv, mask=None, drop_m
     _req(dctx, torch.bfloat16, "dctx")
     _req(ctx, torch.bfloat16, "ctx")
     W = q.shape[-1]
+    _shape(dctx, (B * Sq, W), "attention_bwd: dctx")
+    _shape(ctx, (B * Sq, W), "attention_bwd: ctx")
+    _req(lse2, torch.float32, "lse2")
+    _shape(lse2, (B, heads, Sq), "attention_bwd: lse2", contiguous=True)
     dq = dq if dq is not None else torch.empty(B * Sq, W, dtype=torch.bfloat16, device=q.device)
     dk = dk if dk is not None else torch.empty(B * Skv, W, dtype=torch.bfloat16, device=q.device)
     dv = dv if dv is not None else torch.empty(B * Skv, W, dtype=torch.bfloat16, device=q.device)
+    for t, n, rows in ((dq, "dq", B * Sq), (dk, "dk", B * Skv), (dv, "dv", B * Skv)):
+        _req(t, torch.bfloat16, n)
+        _shape(t, (rows, W), "attention_bwd: " + n)
     delta = torch.empty(B, heads, Sq, dtype=torch.float32, device=q.device)
     a.ctx, a.ldo, a.lse2 = ctx.data_ptr(), ctx.stride(0), lse2.data_ptr()
     a.dctx, a.ld_dctx, a.delta = dctx.data_ptr(), dctx.stride(0), delta.data_ptr()
     if ctx_lo is not None:
         _req(ctx_lo, torch.bfloat16, "ctx_lo")
-        if not ctx_lo.is_contiguous():
+        if not ctx_lo.is_contiguous() or tuple(ctx_lo.shape) != (B * Sq, W):
             raise ValueError("ctx_lo must be contiguous [B*Sq, heads*head_dim]")
         a.ctx_lo = ctx_lo.data_ptr()
     a.dq, a.ld_dq = dq.data_ptr(), dq.stride(0)
@@ -166,7 +195,11 @@ def layernorm_fwd(y, gamma, beta, eps=LN_EPS, drop_mask=None, drop_scale=1.0, ou
     """x, mean, rstd = LayerNorm(y) over the last dim; y bf16 [M,H] (row stride allowed)."""
     _req(y, torch.bfloat16, "y"); _req(gamma, torch.bfloat16, "gamma"); _req(beta, torch.bfloat16, "beta")
     M, H = y.shape
+    _shape(gamma, (H,), "layernorm_fwd: gamma", contiguous=True)
+    _shape(beta, (H,), "layernorm_fwd: beta", contiguous=True)
     x = out if out is not None else torch.empty(M, H, dtype=torch.bfloat16, device=y.device)
+    _req(x, torch.bfloat16, "out")
+    _shape(x, (M, H), "layernorm_fwd: out")
     mean = torch.empty(M, dtype=torch.float32, device=y.device)
     rstd = torch.empty(M, dtype=torch.float32, device=y.device)
     a = LnArgs()
@@ -174,6 +207,7 @@ def layernorm_fwd(y, gamma, beta, eps=LN_EPS, drop_mask=None, drop_scale=1.0, ou
     a.x, a.ldx, a.mean, a.rstd = x.data_ptr(), x.stride(0), mean.data_ptr(), rstd.data_ptr()
     if drop_mask is not None:
         _req(drop_mask, torch.int32, "drop_mask")
+        _shape(drop_mask, (M, (H + 31) // 32), "layernorm_fwd: drop_mask")
         a.drop_mask, a.ldmask, a.drop_scale = drop_mask.data_ptr(), drop_mask.stride(0), float(drop_scale)
     a.eps, a.M, a.H = float(eps), M, H
     check(LIB.mmfb_layernorm_fwd(ctypes.byref(a), _stream_ptr()))
@@ -187,6 +221,12 @@ def layernorm_bwd(dx, y, mean, rstd, gamma, dgamma, dbeta, dbias=None, dx2=None,
     accumulated in place."""
     _req(dx, torch.bfloat16, "dx"); _req(y, torch.bfloat16, "y"); _req(gamma, torch.bfloat16, "gamma")
     M, H = y.shape
+    _shape(dx, (M, H), "layernorm_bwd: dx")
+    _shape(dx2, (M, H), "layernorm_bwd: dx2")
+    _shape(gamma, (H,), "layernorm_bwd: gamma", contiguous=True)
+    for name, t in (("mean", mean), ("rstd", rstd)):
+        _req(t, torch.float32, name)
+        _shape(t, (M,), "layernorm_bwd: " + name, contiguous=True)
     dy = torch.empty(M, H, dtype=torch.bfloat16, device=y.device)
     a = LnArgs()
     a.dx, a.lddx = dx.data_ptr(), dx.stride(0)
@@ -198,12 +238,14 @@ def layernorm_bwd(dx, y, mean, rstd, gamma, dgamma, dbeta, dbias=None, dx2=None,
     dz = dy
     if drop_mask is not None:
         _req(drop_mask, torch.int32, "drop_mask")
+        _shape(drop_mask, (M, (H + 31) // 32), "layernorm_bwd: drop_mask")
         dz = torch.empty(M, H, dtype=torch.bfloat16, device=y.device)
         a.drop_mask, a.ldmask, a.drop_scale = drop_mask.data_ptr(), drop_mask.stride(0), float(drop_scale)
     a.dz, a.lddz = dz.data_ptr(), dz.stride(0)
     for name, t in (("dgamma", dgamma), ("dbeta", dbeta), ("dbias", dbias)):
         if t is not None:
             _req(t, torch.float32, name)
+            _shape(t, (H,), "layernorm_bwd: " + name, contiguous=True)
             setattr(a, name, t.data_ptr())
     a.M, a.H = M, H
     check(LIB.mmfb_layernorm_bwd(ctypes.byref(a), _stream_ptr()))
@@ -268,6 +310,7 @@ def ce_rows(logits, labels, ignore_index, grad_scale, loss_sum, row_loss=None):
     rl = None
     if row_loss is not None:
         _req(row_loss, torch.float32, "row_loss")
+        _shape(row_loss, (M,), "ce_rows: row_loss", contiguous=True)
         rl = row_loss.data_ptr()
     check(LIB.mmfb_ce_rows(logits.data_ptr(), logits.stride(0), labels.data_ptr(), int(ignore_index), M, V, float(grad_scale),
                            loss_sum.data_ptr(), rl, _stream_ptr()))

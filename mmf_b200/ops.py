@@ -244,8 +244,15 @@ class _LinearCrossEntropy(torch.autograd.Function):
             bb = torch.cat([bb, torch.full((pad,), -30000.0, dtype=torch.bfloat16, device=bb.device)])
         M = hb.shape[0]
         labels = labels.reshape(-1).to(torch.int64).contiguous()
-        n_active = (labels != ignore_index).sum()
-        scale = 1.0 / float(max(int(n_active), 1))      # the one host read of the head (the reference's mean reduction)
+        # the one host read of the head (the reference's mean reduction) also carries the count of labels outside [0, V):
+        # the kernel would score a label in the vocabulary padding against a pad column and silently drop a negative one,
+        # where the reference's CrossEntropyLoss raises
+        active = labels != ignore_index
+        n_active, n_bad = torch.stack([active.sum(), (active & ((labels < 0) | (labels >= V))).sum()]).tolist()
+        if n_bad:
+            raise ValueError("linear_cross_entropy: %d label(s) outside [0, %d) that are not ignore_index (%d)"
+                             % (n_bad, V, ignore_index))
+        scale = 1.0 / float(max(n_active, 1))
         loss_sum = torch.zeros((), dtype=torch.float32, device=wb.device)
         need_h, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
         need_b = bias is not None and ctx.needs_input_grad[2]
